@@ -1,7 +1,7 @@
 #!/usr/bin/env python
-"""bench.py -- WCSPH step throughput on B200 (contract: see the task statement / DESIGN.md section 6).
+"""bench.py -- WCSPH step throughput on B200 (see DESIGN.md section 6).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--scene NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--scene NAME] [--dump-outputs DIR]
 
 One "step" is one full ``SPHBase.step()`` (neighbour build + density + forces + integration +
 walls, sph_base.py:263-271 of the reference) over the named scene.  N = 1 runs BASELINE config 2
@@ -13,6 +13,10 @@ flushed between timed steps; ``steady`` = back-to-back steps (state L2-resident,
 simulation actually runs); ``e2e`` = the same through the public Python surface with pinned HOST
 buffers (H2D of x, v and D2H of x, v every step); ``roofline`` for the force kernel;
 ``cpu_baseline`` = the CPU oracle port on this box's cores (bounded sample).
+
+``--dump-outputs DIR`` (single GPU) writes the state after the last of the K L2-flushed timed steps of the first
+measurement, i.e. after W + 3 + K steps from the scene's initial lattice, as DIR/{x,v,density,pressure}.npy
+(float32, see ``step_outputs``): two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -326,6 +330,33 @@ def run_reference(args):
     return 0
 
 
+DUMP_FIELDS = ("x", "v", "density", "pressure")
+DUMP_MAX_BYTES = 64 * 10 ** 6
+
+
+def step_outputs(ps):
+    """What a caller of the stepped ParticleSystem reads back -- positions, velocities, densities, pressures -- as
+    float32 arrays with one row per particle.  The neighbour sort reorders particles, so rows are put in a fixed
+    order: by object id, then rest position x_0.  If all rows exceed DUMP_MAX_BYTES, a seeded random subset of them
+    (the same for every run of the scene) is kept."""
+    import numpy as np
+    x0, oid = ps.x_0.to_numpy(), ps.object_id.to_numpy()
+    rows = np.lexsort((x0[:, 2], x0[:, 1], x0[:, 0], oid))
+    out = {f: getattr(ps, f).to_numpy().astype(np.float32) for f in DUMP_FIELDS}
+    row_bytes = sum(a[0].nbytes for a in out.values())
+    keep = (DUMP_MAX_BYTES - 128 * len(out)) // row_bytes  # 128: the .npy header of each file
+    if len(rows) > keep:
+        rows = rows[np.sort(np.random.default_rng(0).choice(len(rows), keep, replace=False))]
+    return {f: np.ascontiguousarray(a[rows]) for f, a in out.items()}
+
+
+def write_outputs(outputs, out_dir):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def pair_work(grid_ids, fluid_mask, grid_num, accepted_pairs):
     """Compute-side work of ONE pass over the neighbourhood (SURVEY.md section 8d): candidate distance
     tests = sum over fluid particles of the population of their 27-cell neighbourhood (cells outside the
@@ -384,6 +415,8 @@ def run_single(args):
         torch.cuda.synchronize()
         launches = eng.launch_count() - launches0
         cold_ms = sum(a.elapsed_time(b) for a, b in ev)
+        if attempt == 0 and args.dump_outputs:  # a re-measurement must not change which state is dumped
+            outputs = step_outputs(ps)
         # ---- steady state: K back-to-back steps (state stays in L2, as in a real run) ----
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         torch.cuda.synchronize()
@@ -494,6 +527,8 @@ def run_single(args):
         "extra_configs": extra,
         "cpu_baseline": cpu,
     }
+    if args.dump_outputs:
+        write_outputs(outputs, args.dump_outputs)
     print(json.dumps(line))
     return 0
 
@@ -540,7 +575,13 @@ def main():
     ap.add_argument("--warmup", type=int, default=50)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--scene", default=None)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the state after the last timed step as DIR/<field>.npy (single GPU only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.gpus != 1 or int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        ap.error("--dump-outputs is implemented for the single-GPU run (--impl b200 --gpus 1)")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

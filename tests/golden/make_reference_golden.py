@@ -83,8 +83,15 @@ SCENES = {
     "dfsph_bodies": (dict(Configuration=base_cfg(method=4, dt=0.004),
                           FluidBlocks=[fluid([0.10, 0.06, 0.10], (6, 6, 6), (0.0, -1.0, 0.0))],
                           RigidBodies=[body(1, (4, 3, 4), (6, 10, 6), True, (0.3, -2.0, 0.0), 600.0)]), 3),
+    # the scene tests/integration/bind_reference_to_emulated_lib.py replays through the C ABI (TRAJECTORY below)
+    "wcsph_binding": (dict(Configuration=base_cfg(),
+                           FluidBlocks=[fluid([0.10, 0.06, 0.10], (6, 7, 6), (0.5, -1.0, 0.0))],
+                           RigidBlocks=[block(1, [0.23, 0.06, 0.10], (3, 5, 6), False)]), 6),
 }
 SMALL = ("wcsph_cube8k",)
+# these also keep the initial colours and x_0 / x / v / density after EVERY step (step_* arrays, one row per step)
+TRAJECTORY = ("wcsph_binding",)
+STEP_FIELDS = ("x_0", "x", "v", "density")
 FIELDS = ("object_id", "x_0", "x", "v", "acceleration", "m_V", "m", "density", "pressure", "material", "is_dynamic",
           "grid_ids")
 
@@ -98,7 +105,7 @@ def snapshot(ps, prefix, out):
         out[prefix + "density_adv"] = ps.density_adv.to_numpy()
 
 
-def run_reference(scene, steps, allow_oob=False):
+def run_reference(scene, steps, allow_oob=False, trajectory=False):
     sys.path.insert(0, os.path.join(HERE, "ti_shim"))
     sys.path.insert(0, REF)
     import taichi as ti
@@ -116,9 +123,17 @@ def run_reference(scene, steps, allow_oob=False):
         solver = ps.build_solver()
         solver.initialize()
         snapshot(ps, "init_", out)
+        if trajectory:
+            out["init_color"] = ps.color.to_numpy()
+        per_step = {f: [] for f in STEP_FIELDS}
         for _ in range(steps):
             solver.step()
+            if trajectory:
+                for f in STEP_FIELDS:
+                    per_step[f].append(getattr(ps, f).to_numpy())
         snapshot(ps, "final_", out)
+        if trajectory:
+            out.update({"step_" + f: np.stack(v) for f, v in per_step.items()})
     os.unlink(path)
     # Particles resting on an UPPER wall sit in the last cell layer, whose +1 neighbours lie outside the grid: the
     # reference reads them unchecked (SURVEY Q3; harmless on Taichi only because the adjacent memory holds zeros).
@@ -141,7 +156,8 @@ if __name__ == "__main__":
     names = args or list(SCENES)
     for name in names:
         scene, steps = SCENES[name]
-        out = run_reference(json.loads(json.dumps(scene)), steps, allow_oob=(name in ("wcsph_walls", "wcsph_dambreak")))
+        out = run_reference(json.loads(json.dumps(scene)), steps, allow_oob=(name in ("wcsph_walls", "wcsph_dambreak")),
+                            trajectory=name in TRAJECTORY)
         # the oracle / engine side reads rigid bodies from a lattice fixture instead of a mesh
         mine = json.loads(json.dumps(scene))
         for k, b in enumerate(mine.get("RigidBodies", [])):

@@ -64,21 +64,5 @@ def test_oracle_reproduces_the_reference_source(name):
 
 def test_reference_goldens_cover_both_solvers_and_rigid_bodies():
     assert {"wcsph_blocks", "wcsph_walls", "wcsph_bodies", "wcsph_dambreak", "dfsph_blocks"} <= set(NAMES)
-
-
-def test_committed_goldens_regenerate_from_the_reference(tmp_path):
-    """Where the reference tree is mounted: re-running the generator reproduces a committed file bit for bit,
-    i.e. the vectors really are what the reference's source computes under the stand-in."""
-    import subprocess
-    import sys
-    if not os.path.isdir("/root/reference"):
-        pytest.skip("reference tree not mounted")
-    res = subprocess.run([sys.executable, os.path.join(GOLD, "make_reference_golden.py"), "--out", str(tmp_path),
-                          "wcsph_walls"], capture_output=True, text=True, timeout=600)
-    assert res.returncode == 0, res.stdout[-1500:] + res.stderr[-1500:]
-    new = np.load(os.path.join(str(tmp_path), "ref_wcsph_walls.npz"))
-    old = np.load(os.path.join(GOLD, "ref_wcsph_walls.npz"))
-    assert set(new.files) == set(old.files)
-    for k in old.files:
-        assert np.array_equal(new[k], old[k]), k
-    assert int(old["oob_cell_reads"]) > 0  # SURVEY Q3, observed: upper-wall contacts read outside the grid
+    # SURVEY Q3, observed when the vectors were made: upper-wall contacts read outside the grid
+    assert int(np.load(os.path.join(GOLD, "ref_wcsph_walls.npz"))["oob_cell_reads"]) > 0

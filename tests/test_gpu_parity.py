@@ -380,7 +380,7 @@ def test_slab_mode_single_rank_equals_plain_engine():
 def test_slab_two_gpus_equals_single_gpu():
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     for graph in (False, True):  # asynchronous launches (default) and CUDA-graph replay with the NCCL group captured
         out = _run_slab_check(2, ["--counts", "64", "24", "24", "--steps", "60"], graph=graph)
         assert out["ok"] and out["migrated"] and all(h > 0 for h in out["halo_bytes"]), (graph, out)
