@@ -18,19 +18,21 @@ sys.path.insert(0, os.path.join(ROOT, "tests", "emu"))
 FAST = ("neighbor_build_bit_exact or per_kernel_parity_mixed_scene or wall_clamp or overflow_path or "
         "stale_grid or out_of_grid or rigid_solve_recovers or random_scatter or (prefix_sum and not 200000) or "
         "dfsph_per_kernel_parity or dfsph_kernels_on_overfull or "
-        "(reproduces_the_reference_source and (blocks or walls or bodies) and not dfsph)")
+        "(reproduces_the_reference_source and (blocks or walls or bodies) and not dfsph) or "
+        "(fp64 and (base or close_pairs or cell_zero or win_cap or count_cut)) or loop_controls[max_iterations_1]")
 ASAN = ("neighbor_build_bit_exact or per_kernel_parity_mixed_scene or wall_clamp or overflow_path or "
         "rigid_solve_recovers or random_scatter or (prefix_sum and not 200000) or dfsph_per_kernel_parity or "
-        "(reproduces_the_reference_source and (walls or bodies))")
+        "(reproduces_the_reference_source and (walls or bodies)) or (fp64 and (base or close_pairs))")
 
 
-def _run(lib, extra_env=None, select=FAST, at_least=14):
+def _run(lib, extra_env=None, select=FAST, at_least=25):
     env = dict(os.environ, SPH_EMU_LIB=lib, PYTHONPATH=ROOT)
     env.pop("SPH_B200_LIB", None)
     env.update(extra_env or {})
     cmd = [sys.executable, "-m", "pytest", "-q", "-x", "-m", "gpu", "-p", "no:cacheprovider", "-k", select,
            os.path.join(ROOT, "tests", "test_gpu_parity.py"), os.path.join(ROOT, "tests", "test_gpu_dfsph.py"),
-           os.path.join(ROOT, "tests", "test_gpu_reference_golden.py")]
+           os.path.join(ROOT, "tests", "test_gpu_reference_golden.py"),
+           os.path.join(ROOT, "tests", "test_gpu_kernel_edges.py")]
     res = subprocess.run(cmd, capture_output=True, text=True, timeout=900, env=env, cwd=ROOT)
     tail = res.stdout[-3000:] + res.stderr[-3000:]
     assert res.returncode == 0, tail
@@ -52,4 +54,4 @@ def test_gpu_parity_subset_under_address_sanitizer():
     if not os.path.isabs(asan_rt) or not os.path.exists(asan_rt):
         pytest.skip("libasan not available")
     lib = build_emu.build(asan=True)
-    _run(lib, {"LD_PRELOAD": asan_rt, "ASAN_OPTIONS": "detect_leaks=0"}, select=ASAN, at_least=11)
+    _run(lib, {"LD_PRELOAD": asan_rt, "ASAN_OPTIONS": "detect_leaks=0"}, select=ASAN, at_least=17)
